@@ -40,6 +40,26 @@ WORKLOADS = {
 }
 
 
+DUMP_MAX_ELEMS = 1 << 20      # per array: larger outputs are dumped as a fixed seeded sample of this many entries (<= 64 MB in all)
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: each array as <out_dir>/<name>.npy (float32, float64 kept); an array of more than DUMP_MAX_ELEMS entries is
+    replaced by its entries at a sorted sample of flat indices seeded by the name, the same in every run, so that two builds can be
+    compared output for output."""
+    import zlib
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = torch.as_tensor(a).detach().reshape(-1).cpu()
+        a = a.double() if a.dtype == torch.float64 else a.float()
+        if a.numel() > DUMP_MAX_ELEMS:
+            g = torch.Generator().manual_seed(zlib.crc32(name.encode()))
+            idx = torch.randperm(a.numel(), generator=g)[:DUMP_MAX_ELEMS].sort().values
+            a = a[idx]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.numpy())
+
+
 def load_peaks():
     try:
         with open(os.path.join(ROOT, "MEASURED_PEAKS.json")) as f:
@@ -496,6 +516,13 @@ def run_ours(args):
     e1.record()
     barrier()
     clocks = sampler.stop()
+    if args.dump_outputs:          # what the last timed step returned: its loss, render, sample count and updated parameters
+        # every rank exports: under the sharded optimizers export_reference_state() gathers the colour masters (a collective)
+        outputs = {"loss": torch.tensor([tr.read_loss()], dtype=torch.float64), "image": tr.image, "weights_sum": tr.weights_sum,
+                   "depth": tr.depth, "num_samples": tr.counters[1:2], **tr.export_reference_state()}
+        if rank == 0:
+            dump_outputs(args.dump_outputs, outputs)
+        del outputs
     ms = torch.tensor([e0.elapsed_time(e1)], device="cuda")
     samples = m_total.clone().float()
     if world > 1:
@@ -663,6 +690,10 @@ def run_stage1(args):
     e1.record()
     torch.cuda.synchronize()
     ms = e0.elapsed_time(e1) / K
+    if args.dump_outputs:          # what the last timed step returned: its loss, image, coverage and updated parameters
+        dump_outputs(args.dump_outputs, {"loss": torch.tensor([s1.read_loss()], dtype=torch.float64), "image": s1.image,
+                                         "weights_sum": s1.weights_sum, "covered_pixels": s1.counters[1:2], "vertex_offsets": s1.offsets,
+                                         **t0.export_reference_state()})
     # rasterize + points alone
     r0, r1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     r0.record()
@@ -735,7 +766,11 @@ def main():
     ap.add_argument("--dp", default="auto", choices=["auto", "nvls", "peer", "nccl"],
                     help="N > 1: 'nvls' = reduce-scatter inside the NVSwitch (multimem) + sharded Adam + multicast all-gather, 'peer' = the "
                          "same with P2P loads / stores over NVLink, 'nccl' = all-reduce + replicated Adam, 'auto' = first that sets up")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed to DIR/<name>.npy (float32 / float64)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU arms")
     if args.impl == "reference":
         run_reference(args)
     elif args.workload == "lego_stage1":

@@ -45,6 +45,22 @@ def march_case(name):
 
 
 MARCH_CASES = ["lego_converged", "lego_cold", "lego_mid", "garden_cascades", "contract", "bound1p5"]
+INFERENCE_CASES = ["lego_converged", "garden_cascades", "contract"]
+# degenerate rays appended to a march case's rays for near_far: axis-parallel (zero components) and guaranteed misses
+NEAR_FAR_EXTRA_O = [[0.0, 0.0, 3.0], [5.0, 5.0, 5.0], [0.2, 0.1, 0.0]]
+NEAR_FAR_EXTRA_D = [[0.0, 0.0, -1.0], [1.0, 0.0, 0.0], [0.0, 1.0, 0.0]]
+PACKBITS_THRESH = [0.0, 0.37, 10.0]
+
+
+def packbits_morton_flatten_case():
+    """-> (density grid [2, 64^3], morton coordinates [5000, 3] int32, rays [300, 2] int32 (offset, count))"""
+    g = torch.Generator().manual_seed(0)
+    grid = torch.rand(2, 64 ** 3, generator=g) * 2 - 0.5
+    grid[0, :100] = -1.0
+    coords = torch.randint(0, 128, (5000, 3), generator=g, dtype=torch.int32)
+    cnt = torch.randint(0, 50, (300,), generator=g)
+    off = torch.cumsum(cnt, 0) - cnt
+    return grid, coords, torch.stack([off, cnt], -1).int()
 
 
 def grid_case(name):

@@ -25,21 +25,3 @@ def pytest_collection_modifyitems(config, items):
     for item in items:
         if "gpu" in item.keywords:
             item.add_marker(skip)
-
-
-@pytest.fixture(scope="session")
-def ref_raymarching():
-    from oracle.build_ref import load_ref
-    return load_ref("_ref_raymarching")
-
-
-@pytest.fixture(scope="session")
-def ref_gridencoder():
-    from oracle.build_ref import load_ref
-    return load_ref("_ref_gridencoder")
-
-
-@pytest.fixture(scope="session")
-def ref_shencoder():
-    from oracle.build_ref import load_ref
-    return load_ref("_ref_shencoder")

@@ -1,7 +1,10 @@
-"""GPU parity: nerf2mesh_b200.raymarching (through the C ABI) vs the reference's own CUDA kernels
-(oracle/_ref) on identical inputs.  Bar: bit-exact sample counts, M, and per-ray sample values
-(integers AND floats -- the arithmetic is reproduced op for op); composite is bit-exact too."""
-import numpy as np
+"""GPU parity: nerf2mesh_b200.raymarching (through the C ABI) vs the reference's own CUDA kernels on identical inputs, through
+their outputs stored under tests/golden/ (reference_ops.json: digests of the reference's outputs, tests/golden/make_golden.py).
+Bar: bit-exact sample counts, M, and per-ray sample values (integers AND floats -- the arithmetic is reproduced op for op);
+composite is bit-exact too."""
+import json
+import os
+
 import pytest
 import torch
 
@@ -11,32 +14,34 @@ from nerf2mesh_b200 import raymarching as rm
 
 pytestmark = pytest.mark.gpu
 
+with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_ops.json")) as _f:
+    GOLD = json.load(_f)
+D = refcall.digest
+
 
 def cu(x):
     return x.cuda() if torch.is_tensor(x) else x
 
 
 @pytest.mark.parametrize("name", cases.MARCH_CASES)
-def test_near_far_bit_exact(ref_raymarching, name):
+def test_near_far_bit_exact(name):
     c = cases.march_case(name)
     ro, rd, aabb = cu(c["rays_o"]), cu(c["rays_d"]), cu(c["aabb"])
-    # add degenerate rays: axis-parallel (zero components) and guaranteed misses
-    ro = torch.cat([ro, torch.tensor([[0.0, 0.0, 3.0], [5.0, 5.0, 5.0], [0.2, 0.1, 0.0]], device="cuda")])
-    rd = torch.cat([rd, torch.tensor([[0.0, 0.0, -1.0], [1.0, 0.0, 0.0], [0.0, 1.0, 0.0]], device="cuda")])
-    n0, f0 = refcall.near_far(ref_raymarching, ro, rd, aabb, c["min_near"])
+    ro = torch.cat([ro, torch.tensor(cases.NEAR_FAR_EXTRA_O, device="cuda")])
+    rd = torch.cat([rd, torch.tensor(cases.NEAR_FAR_EXTRA_D, device="cuda")])
     n1, f1 = rm.near_far_from_aabb(ro, rd, aabb, c["min_near"])
-    assert torch.equal(n0, n1) and torch.equal(f0, f1)
+    g = GOLD[f"near_far/{name}"]
+    assert D(n1) == g["nears"] and D(f1) == g["fars"]
 
 
 @pytest.mark.parametrize("name", cases.MARCH_CASES)
-def test_march_rays_train_bit_exact(ref_raymarching, name):
+def test_march_rays_train_bit_exact(name):
     c = cases.march_case(name)
+    g = GOLD[f"march_train/{name}"]
     ro, rd, bits, aabb = cu(c["rays_o"]), cu(c["rays_d"]), cu(c["bits"]), cu(c["aabb"])
     nears, fars = rm.near_far_from_aabb(ro, rd, aabb, c["min_near"])
     noises = cu(c["noises"])
-    x0, d0, t0, r0 = refcall.march_train(ref_raymarching, ro, rd, bits, c["bound"], c["contract"], c["dt_gamma"],
-                                         c["max_steps"], c["C"], c["H"], nears, fars, noises)
-    # ours, with the wrapper's RNG replaced by the same noises: call the C ABI protocol directly
+    # the wrapper's RNG replaced by the same noises: call the C ABI protocol directly
     from nerf2mesh_b200._lib import call, ptr, stream
     N = ro.shape[0]
     for use_slab in (True, False):
@@ -47,18 +52,17 @@ def test_march_rays_train_bit_exact(ref_raymarching, name):
                 c["C"], c["H"], ptr(nears), ptr(fars))
         call("n2m_march_rays_train", *args, None, None, None, ptr(rays), ptr(counter), ptr(noises), ptr(tbuf), stream())
         M = int(counter.item())
-        assert M == x0.shape[0], f"M differs: {M} vs {x0.shape[0]}"
+        assert M == g["M"], f"M differs: {M} vs {g['M']}"
         assert M > 0
         # counts bit-exact; our offsets are the exclusive scan in ray order
-        assert torch.equal(rays[:, 1], r0[:, 1])
+        assert D(rays[:, 1]) == g["counts"]
         cnt = rays[:, 1].long()
         assert torch.equal(rays[:, 0].long(), torch.cumsum(cnt, 0) - cnt)
         x1 = torch.zeros(M, 3, device="cuda"); d1 = torch.zeros(M, 3, device="cuda"); t1 = torch.zeros(M, 2, device="cuda")
         call("n2m_march_rays_train", *args, ptr(x1), ptr(d1), ptr(t1), ptr(rays), ptr(counter), ptr(noises), ptr(tbuf), stream())
         torch.cuda.synchronize()
-        for a, b, nm in ((x0, x1, "xyzs"), (d0, d1, "dirs"), (t0, t1, "ts")):
-            ra = refcall.by_ray(a, r0); rb = refcall.by_ray(b, rays)
-            assert np.array_equal(ra, rb), f"{nm} differ (slab={use_slab}): max abs {np.abs(ra - rb).max()}"
+        for b, nm in ((x1, "xyzs"), (d1, "dirs"), (t1, "ts")):
+            assert D(refcall.by_ray(b, rays)) == g[nm], f"{nm} differ (slab={use_slab})"
 
 
 def test_march_wrapper_matches_abi():
@@ -80,118 +84,66 @@ def test_march_wrapper_matches_abi():
 
 @pytest.mark.parametrize("alpha_mode", [False, True])
 @pytest.mark.parametrize("T_thresh", [1e-4, 1e-2])
-def test_composite_train_bit_exact(ref_raymarching, alpha_mode, T_thresh):
+def test_composite_train_bit_exact(alpha_mode, T_thresh):
     c = cases.composite_case()
+    g = GOLD[f"composite/{alpha_mode}/{T_thresh}"]
     sig = cu(c["sigmas"]); rgb = cu(c["rgbs"]); ts = cu(c["ts"]); rays = cu(c["rays"])
     if alpha_mode:
         sig = (sig / sig.max()).clamp(0, 0.999)
-    w0, ws0, d0, i0 = refcall.composite_fwd(ref_raymarching, sig, rgb, ts, rays, T_thresh, alpha_mode)
     w1, ws1, d1, i1 = rm.composite_rays_train(sig, rgb, ts, rays, T_thresh, alpha_mode)
-    for a, b in ((w0, w1), (ws0, ws1), (d0, d1), (i0, i1)):
-        assert torch.equal(a, b)
+    for b, k in ((w1, "w"), (ws1, "ws"), (d1, "d"), (i1, "im")):
+        assert D(b) == g[k], k
     gw, gws, gd, gi = cu(c["grad_weights"]), cu(c["grad_weights_sum"]), cu(c["grad_depth"]), cu(c["grad_image"])
-    gs0, gr0 = refcall.composite_bwd(ref_raymarching, gw, gws, gd, gi, sig, rgb, ts, rays, ws0, d0, i0, T_thresh, alpha_mode)
     sig_r = sig.clone().requires_grad_(True); rgb_r = rgb.clone().requires_grad_(True)
     w, ws, d, im = rm.composite_rays_train(sig_r, rgb_r, ts, rays, T_thresh, alpha_mode)
     torch.autograd.backward([w, ws, d, im], [gw, gws, gd, gi])
-    assert torch.equal(sig_r.grad, gs0) and torch.equal(rgb_r.grad, gr0)
+    assert D(sig_r.grad) == g["gs"] and D(rgb_r.grad) == g["gr"]
 
 
-def test_composite_rays_beyond_M_zeroed(ref_raymarching):
+def test_composite_rays_beyond_M_zeroed():
     """rays whose slice exceeds M produce zeros (raymarching.cu:521-528)."""
     c = cases.composite_case(N=16)
+    g = GOLD["composite_beyond_M"]
     sig = cu(c["sigmas"]); rgb = cu(c["rgbs"]); ts = cu(c["ts"]); rays = cu(c["rays"]).clone()
     rays[-1, 1] += 1000
-    w0, ws0, d0, i0 = refcall.composite_fwd(ref_raymarching, sig, rgb, ts, rays, 1e-4, False)
     w1, ws1, d1, i1 = rm.composite_rays_train(sig, rgb, ts, rays, 1e-4, False)
-    assert torch.equal(ws0, ws1) and torch.equal(i0, i1) and torch.equal(w0, w1)
+    assert D(ws1) == g["ws"] and D(i1) == g["im"] and D(w1) == g["w"]
     assert ws1[-1] == 0
 
 
-@pytest.mark.parametrize("name", ["lego_converged", "garden_cascades", "contract"])
-def test_inference_loop_bit_exact(ref_raymarching, name):
-    """The eval loop of renderer.py:764-802 driven with both backends on identical sigmas/rgbs."""
-    c = cases.march_case(name)
-    ro, rd, bits, aabb = cu(c["rays_o"]), cu(c["rays_d"]), cu(c["bits"]), cu(c["aabb"])
-    N = ro.shape[0]
-    nears, fars = rm.near_far_from_aabb(ro, rd, aabb, c["min_near"])
-
-    def field(xyzs):       # deterministic stand-in for the network
-        s = (xyzs.sum(-1) * 37.0).sin().abs() * 30.0
-        return s, (xyzs * 0.5 + 0.5).clamp(0, 1)
-
-    outs = []
-    for backend in ("ref", "ours"):
-        ws = torch.zeros(N, device="cuda"); depth = torch.zeros(N, device="cuda"); image = torch.zeros(N, 3, device="cuda")
-        alive = torch.arange(N, dtype=torch.int32, device="cuda"); rays_t = nears.clone()
-        step = 0
-        trace = []
-        while step < 256:
-            n_alive = alive.shape[0]
-            if n_alive <= 0:
-                break
-            n_step = max(min(N // n_alive, 8), 1)
-            if backend == "ref":
-                M = n_alive * n_step
-                xyzs = torch.zeros(M, 3, device="cuda"); dirs = torch.zeros(M, 3, device="cuda"); ts = torch.zeros(M, 2, device="cuda")
-                noises = torch.zeros(n_alive, device="cuda")
-                ref_raymarching.march_rays(n_alive, n_step, alive, rays_t, ro, rd, c["bound"], c["contract"], c["dt_gamma"],
-                                           c["max_steps"], c["C"], c["H"], bits, nears, fars, xyzs, dirs, ts, noises)
-                s, col = field(xyzs)
-                ref_raymarching.composite_rays(n_alive, n_step, 1e-2, False, alive, rays_t, s, col, ts, ws, depth, image)
-            else:
-                xyzs, dirs, ts = rm.march_rays(n_alive, n_step, alive, rays_t, ro, rd, c["bound"], c["contract"], bits,
-                                               c["C"], c["H"], nears, fars, False, c["dt_gamma"], c["max_steps"])
-                s, col = field(xyzs)
-                rm.composite_rays(n_alive, n_step, alive, rays_t, s, col, ts, ws, depth, image, 1e-2, False)
-            trace.append((xyzs.clone(), ts.clone()))
-            alive = alive[alive >= 0]
-            step += n_step
-        outs.append((ws, depth, image, rays_t, trace))
-    a, b = outs
-    assert len(a[4]) == len(b[4])
-    for (xa, ta), (xb, tb) in zip(a[4], b[4]):
-        assert torch.equal(xa, xb) and torch.equal(ta, tb)
-    for k in range(4):
-        assert torch.equal(a[k], b[k])
+@pytest.mark.parametrize("name", cases.INFERENCE_CASES)
+def test_inference_loop_bit_exact(name):
+    """The eval loop of renderer.py:764-802 driven with our operators on the sigmas / rgbs the reference's loop saw."""
+    g = GOLD[f"inference/{name}"]
+    ws, depth, image, rays_t, trace = refcall.inference_loop(cases.march_case(name))
+    assert len(trace) == g["rounds"]
+    assert refcall.trace_digest(trace) == g["trace"]          # every round's samples
+    for a, k in ((ws, "ws"), (depth, "depth"), (image, "image"), (rays_t, "rays_t")):
+        assert D(a) == g[k], k
 
 
-def test_packbits_morton_flatten_exact(ref_raymarching):
-    g = torch.Generator().manual_seed(0)
-    grid = torch.rand(2, 64 ** 3, generator=g).cuda() * 2 - 0.5
-    grid[0, :100] = -1.0
-    for thresh in (0.0, 0.37, 10.0):
-        b0 = torch.empty(grid.numel() // 8, dtype=torch.uint8, device="cuda")
-        ref_raymarching.packbits(grid, grid.numel() // 8, thresh, b0)
+def test_packbits_morton_flatten_exact():
+    g = GOLD["packbits_morton_flatten"]
+    grid, coords, rays = cases.packbits_morton_flatten_case()
+    grid, coords, rays = grid.cuda(), coords.cuda(), rays.cuda()
+    for thresh in cases.PACKBITS_THRESH:
         b1 = rm.packbits(grid, thresh)
-        assert torch.equal(b0, b1)
+        assert D(b1) == g[f"packbits/{thresh}"]
         # in-place variant + unaligned view
         buf = torch.zeros(grid.numel() // 8 + 8, dtype=torch.uint8, device="cuda")
         out = rm.packbits(grid, thresh, buf[1:1 + grid.numel() // 8])
-        assert torch.equal(out, b0)
-    coords = torch.randint(0, 128, (5000, 3), generator=g, dtype=torch.int32).cuda()
-    i0 = torch.empty(5000, dtype=torch.int32, device="cuda")
-    ref_raymarching.morton3D(coords, 5000, i0)
+        assert torch.equal(out, b1)
     i1 = rm.morton3D(coords)
-    assert torch.equal(i0, i1)
+    assert D(i1) == g["morton3D"]
     c1 = rm.morton3D_invert(i1)
     assert torch.equal(c1, coords)
-    c0 = torch.empty(5000, 3, dtype=torch.int32, device="cuda")
-    ref_raymarching.morton3D_invert(i0, 5000, c0)
-    assert torch.equal(c0, c1)
-    cnt = torch.randint(0, 50, (300,), generator=g)
-    off = torch.cumsum(cnt, 0) - cnt
-    rays = torch.stack([off, cnt], -1).int().cuda()
-    M = int(cnt.sum())
-    f0 = torch.zeros(M, dtype=torch.int32, device="cuda")
-    ref_raymarching.flatten_rays(rays, 300, M, f0)
-    assert torch.equal(f0, rm.flatten_rays(rays, M))
+    assert D(c1) == g["morton3D_invert"]
+    assert D(rm.flatten_rays(rays, int(rays[:, 1].sum()))) == g["flatten_rays"]
 
 
-def test_sph_from_ray_close(ref_raymarching):
+def test_sph_from_ray_close():
     ro, rd = cases.rays(500, seed=9)
     ro, rd = ro.cuda() * 0.2, rd.cuda()
-    c0 = torch.empty(500, 2, device="cuda")
-    ref_raymarching.sph_from_ray(ro, rd, 4.0, 500, c0)
+    c0 = torch.tensor(GOLD["sph_from_ray"], device="cuda")
     c1 = rm.sph_from_ray(ro, rd, 4.0)
     assert torch.allclose(c0, c1, atol=1e-6, rtol=0)

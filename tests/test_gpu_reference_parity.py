@@ -1,10 +1,15 @@
-"""Parity of the BENCHMARKED path -- one fused 4096-ray train step (Stage0Trainer) -- against the reference's OWN CUDA path:
-the unmodified nerf/network.py + nerf/renderer.py + nerf/utils.py (Trainer.train_step / post_train_step) over the unmodified
-raymarching / gridencoder wrappers and the reference's kernels compiled for sm_100a (oracle/ref_stage.py, oracle/_ref).
+"""Parity of the BENCHMARKED path -- one fused 4096-ray train step (Stage0Trainer) -- and of the code around it against the reference's
+OWN CUDA path: the unmodified nerf/network.py + nerf/renderer.py + nerf/utils.py (Trainer.train_step / post_train_step) over the
+unmodified raymarching / gridencoder wrappers and the reference's kernels compiled for sm_100a (oracle/ref_stage.py, oracle/_ref).
 
-Both sides start from the same parameters (a few fused warm-up steps away from the initialisation, so that densities, colours
-and gradients are non-trivial), the same rays, ground truth, background colours and march noises (same torch CUDA generator
-state: Trainer.train_step draws bg_color, utils.py:660, then march_rays_train draws the noises, raymarching.py:223).
+The reference's results are stored in tests/golden/reference_model.npz (refcall.Golden: scalars, digests of what must agree bit for
+bit, and for every large tensor its values at stored rows -- a seeded sample, or for the sparse gradient tables a sample of the rows
+where they are non-zero -- with its full-tensor size, max |.| and norm); `reference_outputs()` below regenerates them where the
+reference is available (tests/golden/make_golden.py).  A comparison with a sampled tensor is made on its stored rows.
+
+Both sides start from the same parameters (refcall.seeded_state: a function of a seed alone, with non-trivial densities, colours
+and gradients), the same rays, ground truth, background colours and march noises (same torch CUDA generator state:
+Trainer.train_step draws bg_color, utils.py:660, then march_rays_train draws the noises, raymarching.py:223).
 
 Configurations: BASELINE config 2 (lego recipe, bound 1, dt_gamma 0, RGBA + mask loss) and config 4 (garden recipe, bound 16 =>
 5 cascades, dt_gamma 1/256, per-ray camera near/far, entropy regulariser, TV with 10x outer weight, RGB images), 4096 rays.
@@ -13,9 +18,9 @@ What is asserted
   * sample counts M, per-ray counts, (t, dt) of every sample: bit-exact;
   * sigma / rgb per sample, image, weights_sum, depth, loss: north_star's 1e-3 (relative to the tensor scale);
   * every gradient: the error against the reference's fp16 run must stay within a small multiple of the reference's OWN
-    fp16 quantisation error (|reference fp16 run - reference fp32 run|, measured here) and of its run-to-run spread
-    (two identical reference runs differ through atomic order); the measured numbers go to gpurun_out/parity_<case>.json
-    and are committed under profiles/.
+    fp16 quantisation error (|reference fp16 run - reference fp32 run|) and of its run-to-run spread (two identical reference
+    runs differ through atomic order); the fp16 and fp32 runs are stored at the same rows, and the reference's own two errors were
+    measured on those rows when the data were made.
 """
 import json
 import os
@@ -25,6 +30,7 @@ import pytest
 import torch
 
 import cases
+import refcall
 from nerf2mesh_b200 import synthetic as S
 from nerf2mesh_b200.stage0 import MLP_LAYOUT, Stage0Config, Stage0Trainer
 
@@ -32,18 +38,27 @@ pytestmark = pytest.mark.gpu
 
 N = 4096
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+GOLD_PATH = os.path.join(ROOT, "tests", "golden", "reference_model.npz")
+K_FWD, K_GRAD, K_LEVEL = 192, 192, 128          # stored rows: per forward tensor, per gradient, per hash-grid level
 
 CASES = {
     "lego": dict(bound=1.0, dt_gamma=0.0, lambda_entropy=0.0, radius=S.LEGO_RADIUS, alpha=True, cam_nf=False, cap=160),
     "garden": dict(bound=16.0, dt_gamma=1.0 / 256, lambda_entropy=1e-3, radius=1.2, alpha=False, cam_nf=True, cap=256),
     "garden_notv": dict(bound=16.0, dt_gamma=1.0 / 256, lambda_entropy=1e-3, radius=1.2, alpha=False, cam_nf=True, cap=256, lambda_tv=0.0),
 }
+_GOLD = []
+
+
+def gold():
+    if not _GOLD:
+        _GOLD.append(refcall.Golden(GOLD_PATH))
+    return _GOLD[0]
 
 
 def _ref_stack():
     from oracle import ref_stage
     if not ref_stage.staged():
-        pytest.skip("reference Python files not staged under oracle/_ref/py (build() stages them where /root/reference exists)")
+        pytest.skip("reference Python files not staged under oracle/_ref/py (build() stages them where the reference tree exists)")
     return ref_stage, ref_stage.load("ref")
 
 
@@ -81,17 +96,6 @@ def _make_ours(c, bits, grid):
     tr.set_occupancy(bits, grid)
     tr.use_cam_near_far = c["cam_nf"]
     return tr
-
-
-def _warm_up(tr, c, bricks, steps=40):
-    """a few fused optimizer steps: diffuse first, then full shading (the reference's schedule in miniature)"""
-    for it in range(steps):
-        ro, rd = _batch(c, 100 + it)
-        g = torch.Generator().manual_seed(1000 + it)
-        tr.step(ro, rd, _gt(c, ro, rd, bricks), torch.rand(N, 3, generator=g), torch.rand(N, generator=g),
-                shading="diffuse" if it < steps // 2 else "full", use_graph=False, cam_near_far=_cam_nf(c, ro))
-    torch.cuda.synchronize()
-    assert tr.counters[2].item() == 0, "sample capacity overflow during warm-up"
 
 
 def _ref_trainer(ref_stage, ns, c, state, fp16, loss_scale=None):
@@ -165,30 +169,52 @@ def _cmp(a, r):
                 cos=(torch.dot(a, r) / (a.norm() * r.norm() + 1e-300)).item(), scale=scale)
 
 
-@pytest.mark.parametrize("name", ["lego", "garden", "garden_notv"])
-def test_fused_step_matches_reference_cuda_path(name):
+def _levels(tr):
+    return tr.offsets.cpu().tolist()
+
+
+FWD = ("sigma", "rgb", "image", "ws", "depth")
+SPARSE = ("encoder.embeddings", "encoder_color.embeddings")      # hash-grid tables: most rows receive no gradient in one batch
+
+
+def _grad_names():
+    return list(SPARSE) + [nm for nm, _ in MLP_LAYOUT]
+
+
+def _fused_setup(name):
     c = CASES[name]
-    ref_stage, ns = _ref_stack()
     grid, bits, bricks = _scene(c)
     tr = _make_ours(c, bits, grid)
-    _warm_up(tr, c, bricks)
-    state = tr.export_reference_state()
-
-    # ---------------- the batch under test ----------------
-    seed = 4242
+    refcall.seeded_state(tr)
     ro, rd = _batch(c, 7)
     gt = _gt(c, ro, rd, bricks)
     cnf = _cam_nf(c, ro)
     data = dict(rays_o=ro.cuda(), rays_d=rd.cuda(), index=[0], images=gt.cuda())
     if cnf is not None:
         data["cam_near_far"] = cnf.cuda()
-    torch.manual_seed(seed)
-    bg = torch.rand(N, 3, device="cuda"); noises = torch.rand(N, device="cuda")       # the draws train_step / march_rays_train will make
+    return c, tr, data
 
-    # ---------------- reference: fp16 twice (run-to-run spread), fp32 once (its own quantisation error) ----------------
+
+def _put_runs(G, key, runs, rows):
+    """the reference's fp16 and fp32 runs of one tensor at the same rows, and on those rows its own fp16-vs-fp32 error and
+    run-to-run spread (runs: ref16, ref16_again, ref32)"""
+    G.put(key + "/ref16", runs["ref16"], index=rows); G.put(key + "/ref32", runs["ref32"], index=rows)
+    on = {tag: t.detach().reshape(-1).double().cpu()[rows] for tag, t in runs.items()}
+    e = _cmp(on["ref16"], on["ref32"])
+    G.put(key + "/ref16_vs_ref32", e["rel_l2"]); G.put(key + "/ref16_vs_ref32_cos", e["cos"])
+    G.put(key + "/ref16_run_to_run", _cmp(on["ref16_again"], on["ref16"])["rel_l2"])
+
+
+def _reference_fused_step(G, name):
+    """the reference side of test_fused_step_matches_reference_cuda_path -> G under fused/<name>/"""
+    P = f"fused/{name}/"
+    ref_stage, ns = _ref_stack()
+    c, tr, data = _fused_setup(name)
+    state = tr.export_reference_state()
+    seed = 4242
     # GradScaler dynamics: the reference produces the gradient of every fp16-cast weight / colour table IN fp16 (autocast), so at the
     # initial scale 65536 a 3e5-sample batch overflows and GradScaler halves the scale until it does not (utils.py:1176-1177).  Find
-    # that scale the way the reference would (back-off by 0.5) and run BOTH sides at it.
+    # that scale the way the reference would (back-off by 0.5); the test runs our side at it.
     scale = 65536.0
     for _ in range(16):
         r16a = _ref_step(_ref_trainer(ref_stage, ns, c, state, True, scale), data, seed)
@@ -200,45 +226,19 @@ def test_fused_step_matches_reference_cuda_path(name):
     if c.get("lambda_tv", 1e-8) == 0:      # post_train_step unscales only inside its TV branch (utils.py:803-812): do what scaler.step would
         for run in (r16a, r16b):
             run["grads"] = {k: v / scale for k, v in run["grads"].items()}
-    tr.opt_state[0] = scale
-    # ---------------- ours ----------------
-    tr.slots[tr.cur].load(data["rays_o"], data["rays_d"], data["images"], bg, noises, data.get("cam_near_far"))
-    tr._fill_params(True, c["alpha"])
-    tr.forward_backward()
-    torch.cuda.synchronize()
-    M = int(tr.counters[1].item())
-    g_ours = tr.export_reference_grads()
-    loss_ours = tr.read_loss()
-
-    rep = {"case": name, "rays": N, "samples": M, "config": {k: v for k, v in c.items()}, "loss_scale": scale,
-           "found_inf_ours": float(tr.opt_state[3].item())}
-    assert tr.opt_state[3].item() == 0
-    # ---- integers: bit-exact ----
-    assert tr.counters[2].item() == 0
-    assert M == r16a["M"] == r16b["M"] == r32["M"], (M, r16a["M"], r32["M"])
-    assert torch.equal(tr.rays[:, 1], r16a["rays"][:, 1]), "per-ray sample counts differ"
-    assert torch.equal(tr.recs[:M, 2], r16a["ts"][:, 0]) and torch.equal(tr.recs[:M, 1], r16a["ts"][:, 1]), "(t, dt) differ"
-    rep["per_ray_counts_equal"] = True
-    fw = {}
-    for tag, run in (("ref16", r16a), ("ref16_again", r16b), ("ref32", r32)):
-        fw[tag] = dict(sigma=run["sigma"], rgb=run["rgb"], image=run["image"], ws=run["ws"], depth=run["depth"], loss=run["loss"])
-    ours = dict(sigma=tr.out[:M, 0], rgb=tr.out[:M, 1:], image=tr.image, ws=tr.weights_sum, depth=tr.depth, loss=loss_ours)
-    rep["forward"] = {}
-    for k in ("sigma", "rgb", "image", "ws", "depth"):
-        rep["forward"][k] = {"ours_vs_ref16": _cmp(ours[k], fw["ref16"][k]), "ref16_vs_ref32": _cmp(fw["ref16"][k], fw["ref32"][k]),
-                             "ours_vs_ref32": _cmp(ours[k], fw["ref32"][k]), "ref16_run_to_run": _cmp(fw["ref16_again"][k], fw["ref16"][k])}
-    rep["loss"] = {"ours": loss_ours, "ref16": r16a["loss"], "ref32": r32["loss"], "rel_err_vs_ref16": abs(loss_ours - r16a["loss"]) / abs(r16a["loss"])}
-
-    # ---- gradients ----
-    names = {"encoder.embeddings": "encoder.embeddings", "encoder_color.embeddings": "encoder_color.embeddings"}
-    for nm, _ in MLP_LAYOUT:
-        names[nm] = nm
-    rep["grads"] = {}
-    for nm in names:
-        ga, gb, g32 = r16a["grads"][nm], r16b["grads"][nm], r32["grads"][nm]
-        rep["grads"][nm] = {"ours_vs_ref16": _cmp(g_ours[nm], ga), "ref16_run_to_run": _cmp(gb, ga), "ref16_vs_ref32": _cmp(ga, g32),
-                            "ours_vs_ref32": _cmp(g_ours[nm], g32)}
-    # TV in isolation, same state: reference post_train_step on a zero gradient vs tr.tv() on a zero gradient table
+    assert r16a["M"] == r16b["M"] == r32["M"]
+    G.put(P + "loss_scale", scale); G.put(P + "M", r16a["M"])
+    G.put(P + "counts", refcall.digest(r16a["rays"][:, 1])); G.put(P + "t", refcall.digest(r16a["ts"][:, 0])); G.put(P + "dt", refcall.digest(r16a["ts"][:, 1]))
+    for k in FWD:
+        key = P + f"fwd/{k}"
+        _put_runs(G, key, dict(ref16=r16a[k], ref16_again=r16b[k], ref32=r32[k]), refcall.sample_index(r16a[k].numel(), K_FWD, key))
+    G.put(P + "loss/ref16", r16a["loss"]); G.put(P + "loss/ref32", r32["loss"])
+    for nm in _grad_names():
+        key = P + f"grad/{nm}"
+        runs = dict(ref16=r16a["grads"][nm], ref16_again=r16b["grads"][nm], ref32=r32["grads"][nm])
+        rows = refcall.support_rows(*runs.values(), k=K_GRAD, key=key) if nm in SPARSE else refcall.sample_index(runs["ref32"].numel(), K_GRAD, key)
+        _put_runs(G, key, runs, rows)
+    # TV in isolation, same state: reference post_train_step on a zero gradient
     rt_tv = _ref_trainer(ref_stage, ns, c, state, True, scale)
     for p_ in rt_tv.model.parameters():
         p_.grad = torch.zeros_like(p_)
@@ -265,7 +265,54 @@ def test_fused_step_matches_reference_cuda_path(name):
     rt_tv.scaler = torch.amp.GradScaler("cuda", enabled=False)
     if c.get("lambda_tv", 1e-8) > 0:
         rt_tv.post_train_step()
-    tv_ref = rt_tv.model.encoder.embeddings.grad.reshape(-1).clone()
+    tv_ref = rt_tv.model.encoder.embeddings.grad.reshape(-1)
+    g32 = r32["grads"]["encoder.embeddings"].reshape(-1); g16 = r16a["grads"]["encoder.embeddings"].reshape(-1)
+    offs = _levels(tr)
+    for l in range(16):          # per level: the same rows for every tensor, drawn from the rows where any of them is non-zero
+        sl = slice(offs[l], offs[l + 1])
+        key = P + f"level{l}"
+        rows = refcall.support_rows(g32[sl], g16[sl], tv_ref[sl], k=K_LEVEL, key=key)
+        G.put(key + "/tv_ref", tv_ref[sl], index=rows); G.put(key + "/ref32", g32[sl], index=rows)
+        G.put(key + "/ref16_vs_ref32", _cmp(g16[sl].double().cpu()[rows], g32[sl].double().cpu()[rows])["rel_l2"])
+
+
+@pytest.mark.parametrize("name", ["lego", "garden", "garden_notv"])
+def test_fused_step_matches_reference_cuda_path(name):
+    """One fused train step against the reference's stored results (tests/golden/reference_model.npz) on the seeded parameters.  Every
+    comparison of a sampled tensor -- ours against the reference's fp16 and fp32 runs, and the reference's own fp16-vs-fp32 error and
+    run-to-run spread that set the bounds (measured when the data were made) -- is made on the same stored rows of that tensor."""
+    P = f"fused/{name}/"
+    G = gold()
+    c, tr, data = _fused_setup(name)
+    seed = 4242
+    torch.manual_seed(seed)
+    bg = torch.rand(N, 3, device="cuda"); noises = torch.rand(N, device="cuda")       # the draws train_step / march_rays_train make
+    scale = G[P + "loss_scale"]
+    tr.opt_state[0] = scale
+    tr.slots[tr.cur].load(data["rays_o"], data["rays_d"], data["images"], bg, noises, data.get("cam_near_far"))
+    tr._fill_params(True, c["alpha"])
+    tr.forward_backward()
+    torch.cuda.synchronize()
+    M = int(tr.counters[1].item())
+    g_ours = tr.export_reference_grads()
+    loss_ours = tr.read_loss()
+    assert tr.opt_state[3].item() == 0
+    # ---- integers: bit-exact ----
+    assert tr.counters[2].item() == 0
+    assert M == G[P + "M"], (M, G[P + "M"])
+    assert refcall.digest(tr.rays[:, 1]) == G[P + "counts"], "per-ray sample counts differ"
+    assert refcall.digest(tr.recs[:M, 2]) == G[P + "t"] and refcall.digest(tr.recs[:M, 1]) == G[P + "dt"], "(t, dt) differ"
+
+    def report(key, ours):
+        return {"ours_vs_ref16": G.cmp(key + "/ref16", ours), "ours_vs_ref32": G.cmp(key + "/ref32", ours),
+                "ref16_vs_ref32": {"rel_l2": G[key + "/ref16_vs_ref32"], "cos": G[key + "/ref16_vs_ref32_cos"]},
+                "ref16_run_to_run": {"rel_l2": G[key + "/ref16_run_to_run"]}}
+
+    ours = dict(sigma=tr.out[:M, 0], rgb=tr.out[:M, 1:], image=tr.image, ws=tr.weights_sum, depth=tr.depth)
+    f = {k: report(P + f"fwd/{k}", ours[k]) for k in FWD}
+    r16_loss = G[P + "loss/ref16"]
+    loss = {"ours": loss_ours, "ref16": r16_loss, "ref32": G[P + "loss/ref32"], "rel_err_vs_ref16": abs(loss_ours - r16_loss) / abs(r16_loss)}
+    grads = {nm: report(P + f"grad/{nm}", g_ours[nm]) for nm in _grad_names()}
     g_full_ours = g_ours["encoder.embeddings"].reshape(-1).clone()
     tr.gtable.zero_()
     tr.tv()
@@ -281,33 +328,25 @@ def test_fused_step_matches_reference_cuda_path(name):
     tr.forward_backward(); torch.cuda.synchronize()
     g_data_ours = tr.export_reference_grads()["encoder.embeddings"].reshape(-1).clone()
     tr.cfg.lambda_tv = lam_keep; tr._fill_params(True, c["alpha"])
-    rep["ours_decomposition_by_level"] = []
-    offs = tr.offsets.cpu().tolist()
+    offs = _levels(tr)
+    decomposition = []
     for l in range(16):
         sl = slice(offs[l], offs[l + 1])
         full, full2, parts = g_full_ours[sl].double(), g_full_ours2[sl].double(), (g_data_ours[sl].double() + tv_ours[sl].double())
-        rep["ours_decomposition_by_level"].append({"level": l, "run_to_run_rel": ((full - full2).norm() / full.norm()).item(),
-                                                   "combined_vs_sum_of_parts_rel": ((full - parts).norm() / full.norm()).item()})
-    # per-level breakdown of the density-table gradient (rows of level l: offsets[l] .. offsets[l+1])
-    rep["tv_alone_by_level"] = []
+        decomposition.append({"level": l, "run_to_run_rel": ((full - full2).norm() / full.norm()).item(),
+                              "combined_vs_sum_of_parts_rel": ((full - parts).norm() / full.norm()).item()})
+    # per-level breakdown of the density-table gradient (rows of level l: offsets[l] .. offsets[l+1]) on the level's stored rows
+    by_level = []
     for l in range(16):
-        a, r = tv_ours[offs[l]:offs[l + 1]].double(), tv_ref[offs[l]:offs[l + 1]].double()
-        full_err = (g_full_ours[offs[l]:offs[l + 1]].double() - r32["grads"]["encoder.embeddings"].reshape(-1)[offs[l]:offs[l + 1]].double())
-        rep["tv_alone_by_level"].append({"level": l, "tv_ref_norm": r.norm().item(), "tv_ours_vs_ref_rel": ((a - r).norm() / max(r.norm().item(), 1e-300)).item(),
-                                         "full_err_norm": full_err.norm().item(),
-                                         "full_err_cos_tv": (torch.dot(full_err, r) / (full_err.norm() * r.norm() + 1e-300)).item()})
-    rep["density_grad_by_level"] = []
-    for l in range(16):
-        a, r = g_ours["encoder.embeddings"][offs[l]:offs[l + 1]], r32["grads"]["encoder.embeddings"][offs[l]:offs[l + 1]]
-        r16 = r16a["grads"]["encoder.embeddings"][offs[l]:offs[l + 1]]
-        rep["density_grad_by_level"].append({"level": l, "ours_vs_ref32": _cmp(a, r), "ref16_vs_ref32": _cmp(r16, r)})
-    os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
-    with open(os.path.join(ROOT, "gpurun_out", f"parity_{name}.json"), "w") as f:
-        json.dump(rep, f, indent=1, default=float)
+        sl = slice(offs[l], offs[l + 1])
+        key = P + f"level{l}"
+        a, tv_r = G.take(key + "/tv_ref", tv_ours[sl])
+        fo, r32 = G.take(key + "/ref32", g_full_ours[sl])
+        by_level.append({"level": l, "tv_ref_norm": tv_r.norm().item(), "tv_ours_vs_ref_rel": ((a - tv_r).norm() / max(tv_r.norm().item(), 1e-300)).item(),
+                         "err_norm": (fo - r32).norm().item(), "gnorm": r32.norm().item(), "ref16_vs_ref32_rel": G[key + "/ref16_vs_ref32"]})
 
     # ---- assertions: forward at north_star's 1e-3 of the tensor scale; sigma through exp() of an fp16 value carries one fp16
-    # ulp of its exponent (2^-11 * |h| relative), so its bound is the reference's own fp16-vs-fp32 error, measured above ----
-    f = rep["forward"]
+    # ulp of its exponent (2^-11 * |h| relative), so its bound is the reference's own fp16-vs-fp32 error ----
     assert f["image"]["ours_vs_ref16"]["max_err_of_scale"] <= 1e-3, f["image"]
     assert f["ws"]["ours_vs_ref16"]["max_err_of_scale"] <= 1e-3, f["ws"]
     assert f["depth"]["ours_vs_ref16"]["max_err_of_scale"] <= 1e-3, f["depth"]
@@ -315,23 +354,20 @@ def test_fused_step_matches_reference_cuda_path(name):
     assert f["sigma"]["ours_vs_ref16"]["rel_l2"] <= 1e-3 or \
         f["sigma"]["ours_vs_ref16"]["rel_l2"] <= 1.5 * f["sigma"]["ref16_vs_ref32"]["rel_l2"], f["sigma"]
     assert f["rgb"]["ours_vs_ref32"]["rel_l2"] <= 1.5 * f["rgb"]["ref16_vs_ref32"]["rel_l2"] + 1e-4, f["rgb"]
-    assert rep["loss"]["rel_err_vs_ref16"] <= 1e-3, rep["loss"]
+    assert loss["rel_err_vs_ref16"] <= 1e-3, loss
     # density table: the reference adds its TV term AFTER the data gradient, one fp32 atomicAdd per SAMPLE -- at the coarse levels ~1e5
     # samples share a cell, i.e. the SAME increment of a few ulps of the accumulator is added ~1e5 times and rounds the same way every
     # time, which biases the reference's own TV contribution there by a few per cent (sign depends on the fraction).  Here the run of
     # same-cell lanes is summed first and TV lands on a near-empty accumulator: combined == data-only + TV-only to 3e-6 and run-to-run
-    # 4e-7 (rep["ours_decomposition_by_level"]).  So the density-table gradient is compared per level, allowing 8 % of that level's TV
-    # norm on top of the data tolerance.
-    for e_tv, e_lv in zip(rep["tv_alone_by_level"], rep["density_grad_by_level"]):
-        l = e_tv["level"]
-        sl = slice(offs[l], offs[l + 1])
-        gnorm = r32["grads"]["encoder.embeddings"].reshape(-1)[sl].double().norm().item()
-        data_tol = max(1.5 * e_lv["ref16_vs_ref32"]["rel_l2"], 1e-3) * gnorm
-        assert e_tv["full_err_norm"] <= 0.08 * e_tv["tv_ref_norm"] + data_tol, (l, e_tv, gnorm)
-        assert e_tv["tv_ours_vs_ref_rel"] <= 5e-3 or e_tv["tv_ref_norm"] == 0, (l, e_tv)
-    for e in rep["ours_decomposition_by_level"]:
+    # 4e-7 (`decomposition`).  So the density-table gradient is compared per level, allowing 8 % of that level's TV norm on top of the
+    # data tolerance.
+    for e in by_level:
+        data_tol = max(1.5 * e["ref16_vs_ref32_rel"], 1e-3) * e["gnorm"]
+        assert e["err_norm"] <= 0.08 * e["tv_ref_norm"] + data_tol, e
+        assert e["tv_ours_vs_ref_rel"] <= 5e-3 or e["tv_ref_norm"] == 0, e
+    for e in decomposition:
         assert e["run_to_run_rel"] <= 1e-5 and e["combined_vs_sum_of_parts_rel"] <= 1e-4, e
-    for nm, g in rep["grads"].items():
+    for nm, g in grads.items():
         if nm == "encoder.embeddings":
             assert g["ours_vs_ref32"]["rel_l2"] <= 1e-2 and g["ours_vs_ref32"]["cos"] > 0.9999, (nm, g)
             continue
@@ -403,15 +439,44 @@ def test_unmodified_reference_model_runs_over_the_drop_in_operators():
 # ------------------------------------------------------------------------------------------------
 # around the step: density-grid update, evaluation render, checkpoint hand-off, EMA -- each against the unmodified reference
 # ------------------------------------------------------------------------------------------------
-def _trained_pair(name, fp16=True, ema=False, steps=40):
-    """(ours, reference Trainer over the reference kernels) holding the same, slightly trained parameters"""
+def _seeded(name):
+    """ours, holding the seeded parameters"""
     c = CASES[name]
-    ref_stage, ns = _ref_stack()
     grid, bits, bricks = _scene(c)
     tr = _make_ours(c, bits, grid)
-    _warm_up(tr, c, bricks, steps)
+    refcall.seeded_state(tr)
+    return c, tr, bricks
+
+
+def _seeded_pair(name, fp16=True):
+    """(ours, reference Trainer over the reference kernels) holding the same seeded parameters"""
+    ref_stage, ns = _ref_stack()
+    c, tr, bricks = _seeded(name)
     rt = _ref_trainer(ref_stage, ns, c, tr.export_reference_state(), fp16)
     return c, tr, rt, bricks
+
+
+K_GRID = 2048
+
+
+def _grid_bits(bitfield):
+    """bit i of byte n <-> cell 8n+i (raymarching.cu:279-288)"""
+    shifts = torch.arange(8, device=bitfield.device, dtype=torch.uint8)
+    return ((bitfield[:, None] >> shifts) & 1).reshape(-1).bool()
+
+
+def _reference_density_grid_update(G, name):
+    P = f"density_update/{name}/"
+    c, tr, rt, _ = _seeded_pair(name)
+    for rnd in range(2):                               # the second round exercises the decay of a non-trivial grid
+        torch.manual_seed(77 + rnd)
+        rt.model.update_extra_state()
+        torch.cuda.synchronize()
+        cells = refcall.sample_index(rt.model.density_grid.numel(), K_GRID, P + f"{rnd}/cells")          # one cell set for both
+        G.put(P + f"{rnd}/grid", rt.model.density_grid, index=cells)
+        G.put(P + f"{rnd}/bits", _grid_bits(rt.model.density_bitfield).float(), index=cells)
+        G.put(P + f"{rnd}/mean_density", float(rt.model.mean_density))
+        G.put(P + f"{rnd}/occupancy", _grid_bits(rt.model.density_bitfield).float().mean().item())
 
 
 @pytest.mark.parametrize("name", ["lego", "garden"])
@@ -419,90 +484,158 @@ def test_density_grid_update_matches_reference_update_extra_state(name):
     """SURVEY.md section 8 a10: Stage0Trainer.update_density_grid vs the unmodified NeRFRenderer.update_extra_state
     (renderer.py:1074-1149) over the reference kernels: same parameters, same torch generator state => same jitter per cell.
     The density values agree to the fp16 rounding of the network; the bitfield may then differ only for cells whose density sits
-    within that rounding of the threshold."""
-    c, tr, rt, _ = _trained_pair(name)
-    for rnd in range(2):                               # the second round exercises the decay of a non-trivial grid
-        torch.manual_seed(77 + rnd)
-        rt.model.update_extra_state()
+    within that rounding of the threshold.  Checked on a stored sample of cells (densities and bits of the same cells)."""
+    P = f"density_update/{name}/"
+    G = gold()
+    c, tr, _ = _seeded(name)
+    for rnd in range(2):
         torch.manual_seed(77 + rnd)
         tr.update_density_grid(decay=0.95, density_thresh=10.0)
         torch.cuda.synchronize()
-        g_ref, g = rt.model.density_grid, tr.density_grid
-        scale = g_ref.abs().max().item()
+        g = tr.density_grid
+        scale = G[P + f"{rnd}/grid:absmax"]
         assert scale > 0
-        assert (g - g_ref).abs().max().item() <= 2e-3 * scale, (rnd, (g - g_ref).abs().max().item(), scale)
-        assert abs(tr.mean_density.item() - rt.model.mean_density) <= 1e-4 * abs(rt.model.mean_density)
-        # bit i of byte n <-> cell 8n+i (raymarching.cu:279-288)
-        shifts = torch.arange(8, device="cuda", dtype=torch.uint8)
-        ours_bits = ((tr.density_bitfield[:, None] >> shifts) & 1).reshape(-1).bool()
-        ref_bits = ((rt.model.density_bitfield[:, None] >> shifts) & 1).reshape(-1).bool()
-        thr = min(rt.model.mean_density, 10.0)
-        occ = ref_bits.float().mean().item()
+        gs, g_ref = G.take(P + f"{rnd}/grid", g)
+        assert (gs - g_ref).abs().max().item() <= 2e-3 * scale, (rnd, (gs - g_ref).abs().max().item(), scale)
+        ref_mean = G[P + f"{rnd}/mean_density"]
+        assert abs(tr.mean_density.item() - ref_mean) <= 1e-4 * abs(ref_mean)
+        ours_bits = _grid_bits(tr.density_bitfield)
+        thr = min(ref_mean, 10.0)
+        occ = G[P + f"{rnd}/occupancy"]
         assert 0.001 < occ < 0.999, occ
         # our bitfield is exactly packbits of OUR grid at OUR threshold (the operator is bit-exact, test_gpu_raymarching) ...
         assert torch.equal(ours_bits, (g.reshape(-1) > min(tr.mean_density.item(), 10.0)))
         # ... so it can differ from the reference's only where the reference's density is within the network's fp16 rounding
         # of the threshold
-        mism = ours_bits != ref_bits
-        band = (g_ref.reshape(-1) - thr).abs() <= 4e-3 * thr
+        ob, ref_bits = G.take(P + f"{rnd}/bits", ours_bits.float())
+        mism = ob != ref_bits
+        band = (g_ref - thr).abs() <= 4e-3 * thr
         assert not (mism & ~band).any(), int((mism & ~band).sum().item())
-        frac = mism.float().mean().item()
+        frac = mism.double().mean().item()
         assert frac < 2e-3, (rnd, frac)
+
+
+def _eval_view():
+    from nerf2mesh_b200.train_synthetic import full_image_rays
+    pose = S.orbit_cameras(3, seed=99)[1]
+    ro, rd = full_image_rays(pose, S.lego_intrinsics() / 8, 100, 100)            # a 100 x 100 view (10 000 rays: 3 ragged chunks)
+    bgt = torch.rand(ro.shape[0], 3, generator=torch.Generator().manual_seed(31))
+    return ro.cuda(), rd.cuda(), bgt.cuda()
+
+
+def _reference_evaluation_render(G):
+    P = "eval_render/"
+    c, tr, rt, bricks = _seeded_pair("lego")
+    ro, rd, bgt = _eval_view()
+    rt.model.eval()
+    opt = rt.opt
+    with torch.no_grad():
+        ev = rt.model.render(ro, rd, bg_color=1, perturb=False, **{k: v for k, v in vars(opt).items() if k not in ("bg_color", "perturb")})
+        ev2 = rt.model.render(ro, rd, bg_color=bgt, perturb=False, **{k: v for k, v in vars(opt).items() if k not in ("bg_color", "perturb")})
+    G.put(P + "image", ev["image"], 1536); G.put(P + "depth", ev["depth"], 768); G.put(P + "image_bg", ev2["image"], 1536)
 
 
 def test_evaluation_render_matches_reference_inference_loop():
     """SURVEY.md section 8 f3 / a11: Stage0Trainer.render (march + gather + tcgen05 MLPs + composite in ray chunks, no host loop
     over slabs) vs the unmodified NeRFRenderer.render in eval mode (march_rays / composite_rays slab loop with alive-ray
     compaction, renderer.py:749-802) over the reference kernels, same parameters."""
-    c, tr, rt, bricks = _trained_pair("lego")
-    from nerf2mesh_b200.train_synthetic import full_image_rays
-    pose = S.orbit_cameras(3, seed=99)[1]
-    ro, rd = full_image_rays(pose, S.lego_intrinsics() / 8, 100, 100)            # a 100 x 100 view (10 000 rays: 3 ragged chunks)
-    ro, rd = ro.cuda(), rd.cuda()
-    rt.model.eval()
-    opt = rt.opt
-    with torch.no_grad():
-        ev = rt.model.render(ro, rd, bg_color=1, perturb=False, **{k: v for k, v in vars(opt).items() if k not in ("bg_color", "perturb")})
+    P = "eval_render/"
+    G = gold()
+    c, tr, bricks = _seeded("lego")
+    ro, rd, bgt = _eval_view()
     img, ws, dep = tr.render(ro, rd, bg_color=1.0)
     torch.cuda.synchronize()
-    assert ev["image"].shape == img.shape
+    assert img.shape == (ro.shape[0], 3)
     covered = (ws > 0.5).float().mean().item()
     assert 0.02 < covered < 0.98, covered                                           # the view really shows the object
-    assert (img - ev["image"]).abs().max().item() <= 2e-3, (img - ev["image"]).abs().max().item()
-    assert (img - ev["image"]).abs().mean().item() <= 2e-4
-    assert (dep - ev["depth"]).abs().max().item() <= 2e-3 * ev["depth"].abs().max().item()
+    a, r = G.take(P + "image", img)
+    assert (a - r).abs().max().item() <= 2e-3, (a - r).abs().max().item()
+    assert (a - r).abs().mean().item() <= 2e-4
+    a, r = G.take(P + "depth", dep)
+    assert (a - r).abs().max().item() <= 2e-3 * G[P + "depth:absmax"]
     # per-ray background tensor on a ragged chunk (the last chunk is shorter than num_rays)
-    bgt = torch.rand(ro.shape[0], 3, device="cuda")
     img2, _, _ = tr.render(ro, rd, bg_color=bgt)
-    with torch.no_grad():
-        ev2 = rt.model.render(ro, rd, bg_color=bgt, perturb=False, **{k: v for k, v in vars(opt).items() if k not in ("bg_color", "perturb")})
-    assert (img2 - ev2["image"]).abs().max().item() <= 2e-3
+    a, r = G.take(P + "image_bg", img2)
+    assert (a - r).abs().max().item() <= 2e-3
 
 
-def test_checkpoint_is_accepted_by_the_reference_trainer_and_ema_matches(tmp_path):
-    """SURVEY.md section 8 f1 (EMA) + f4 (hand-off): a checkpoint written by Stage0Trainer.save_reference_checkpoint is read by the
-    UNMODIFIED Trainer.load_checkpoint (nerf/utils.py:1407-1473) without missing / unexpected keys, including the torch_ema state;
-    the reference model then renders the same image; and the fused EMA kernels follow torch_ema step by step."""
-    c, tr, rt, bricks = _trained_pair("lego", steps=24)
-    ref_stage, ns = _ref_stack()
-    # --- EMA: ours vs torch_ema (oracle/torch_ema_port.py unless the real package is installed) on the reference's parameters ---
-    EMA = ns.utils.ExponentialMovingAverage
-    ema_ref = EMA(rt.model.parameters(), decay=0.95)
+def _checkpoint_run(c, tr, bricks, ema):
+    """a few optimizer steps per "epoch" on our side, the parameters mirrored into `ema` (torch_ema's interface) once per epoch"""
     tr.enable_ema(0.95)
     for epoch in range(3):
-        for it in range(4):       # a few optimizer steps per "epoch" on our side, mirrored into the reference's parameters
+        for it in range(4):
             ro, rd = _batch(c, 500 + 10 * epoch + it)
             g = torch.Generator().manual_seed(9000 + 10 * epoch + it)
             tr.step(ro, rd, _gt(c, ro, rd, bricks), torch.rand(N, 3, generator=g), torch.rand(N, generator=g), use_graph=False)
-        rt.model.load_state_dict(tr.export_reference_state(), strict=True)
-        ema_ref.update()          # utils.py:1213-1214: once per epoch
+        ema(tr.export_reference_state())
         tr.ema_update()
+
+
+def _handoff_checkpoint(path):
+    """ours with the seeded parameters and an updated density grid, saved with Stage0Trainer.save_reference_checkpoint"""
+    c, tr, bricks = _seeded("lego")
+    tr.enable_ema(0.95)
+    tr.ema_update()
+    torch.manual_seed(5)
+    tr.update_density_grid()
+    tr.save_reference_checkpoint(str(path), epoch=3, full=True)
+    return tr
+
+
+def _reference_checkpoint(G, tmp_dir):
+    """the reference's checkpoint schema (what the unmodified Trainer.load_checkpoint, nerf/utils.py:1407-1473, reads without a
+    warning) and its render after loading our checkpoint of the seeded parameters"""
+    P = "checkpoint/"
+    ref_stage, ns = _ref_stack()
+    path = os.path.join(tmp_dir, "ngp_stage0_ep0003.pth")
+    _handoff_checkpoint(path)
+    opt = ref_stage.default_opt(bound=1.0, dt_gamma=0.0, adaptive_num_rays=False)
+    fresh = ns.make_model(opt)
+    logs = []
+    rt2 = ns.utils.Trainer("ngp", opt, fresh, device=torch.device("cuda"), workspace=None, mute=True,
+                           optimizer=lambda m: torch.optim.Adam(m.get_params(opt.lr), eps=1e-15),
+                           criterion=torch.nn.MSELoss(reduction="none"), ema_decay=0.95, fp16=True,
+                           use_checkpoint="scratch", use_tensorboardX=False, scheduler_update_every_step=True)
+    rt2.log = lambda *a, **k: logs.append(" ".join(str(x) for x in a))
+    rt2.load_checkpoint(path)                                     # the unmodified loader
+    assert not any("[WARN]" in m for m in logs) and any("loaded EMA" in m for m in logs), logs
+    G.put(P + "state_dict", json.dumps({k: list(v.shape) for k, v in rt2.model.state_dict().items()}))
+    G.put(P + "parameters", json.dumps([[n, list(p.shape)] for n, p in rt2.model.named_parameters()]))
+    ro, rd = cases.rays(2048, seed=21)
+    with torch.no_grad():
+        rt2.model.eval()
+        ev = rt2.model.render(ro.cuda(), rd.cuda(), bg_color=1, perturb=False,
+                              **{k: v for k, v in vars(opt).items() if k not in ("bg_color", "perturb")})
+    G.put(P + "image", ev["image"], 1536)
+
+
+def test_checkpoint_is_accepted_by_the_reference_trainer_and_ema_matches(tmp_path):
+    """SURVEY.md section 8 f1 (EMA) + f4 (hand-off): a checkpoint written by Stage0Trainer.save_reference_checkpoint has the schema the
+    UNMODIFIED Trainer.load_checkpoint (nerf/utils.py:1407-1473) reads without missing / unexpected keys, including the torch_ema state;
+    the reference model loaded from it renders the same image; and the fused EMA kernels follow torch_ema step by step
+    (oracle/torch_ema_port.py, the restatement the reference's Trainer runs with when torch_ema is not installed)."""
+    from oracle.torch_ema_port import ExponentialMovingAverage as EMA
+    P = "checkpoint/"
+    G = gold()
+    c, tr, bricks = _seeded("lego")
+    params = json.loads(G[P + "parameters"])
+    names = [n for n, _ in params]
+    st0 = tr.export_reference_state()
+    mirror = [torch.nn.Parameter(st0[n].clone().cuda()) for n in names]
+    ema_ref = EMA(mirror, decay=0.95)
+
+    def follow(st):           # the reference's parameters hold ours; utils.py:1213-1214: one EMA update per epoch
+        with torch.no_grad():
+            for p, n in zip(mirror, names):
+                p.copy_(st[n])
+        ema_ref.update()
+
+    _checkpoint_run(c, tr, bricks, follow)
     st = tr.ema_state_dict()
     assert st["num_updates"] == ema_ref.num_updates == 3 and st["decay"] == ema_ref.decay
-    names = [n for n, _ in rt.model.named_parameters()]
     assert len(names) == len(st["shadow_params"]) == len(ema_ref.shadow_params)
-    for n, a, b in zip(names, st["shadow_params"], ema_ref.shadow_params):
-        assert a.shape == b.shape, n
+    for (n, shape), a, b in zip(params, st["shadow_params"], ema_ref.shadow_params):
+        assert list(a.shape) == list(b.shape) == shape, n
         assert (a - b).abs().max().item() <= 1e-6 * max(b.abs().max().item(), 1e-12) + 1e-9, n
     # ema_apply / ema_restore == store + copy_to / restore
     before = tr.export_reference_state()
@@ -517,49 +650,42 @@ def test_checkpoint_is_accepted_by_the_reference_trainer_and_ema_matches(tmp_pat
     for k in before:
         assert torch.equal(before[k], after[k]), k
 
-    # --- checkpoint hand-off ---
+    # --- checkpoint hand-off: the schema Trainer.load_checkpoint reads (model without missing / unexpected keys, EMA, mean_density,
+    # stats, epoch, global step) ---
     tr.update_density_grid()
     path = tmp_path / "ngp_stage0_ep0003.pth"
     tr.save_reference_checkpoint(str(path), epoch=3, full=True)
-    opt = ref_stage.default_opt(bound=1.0, dt_gamma=0.0, adaptive_num_rays=False)
-    fresh = ns.make_model(opt)
-    logs = []
-    rt2 = ns.utils.Trainer("ngp", opt, fresh, device=torch.device("cuda"), workspace=None, mute=True,
-                           optimizer=lambda m: torch.optim.Adam(m.get_params(opt.lr), eps=1e-15),
-                           criterion=torch.nn.MSELoss(reduction="none"), ema_decay=0.95, fp16=True,
-                           use_checkpoint="scratch", use_tensorboardX=False, scheduler_update_every_step=True)
-    rt2.log = lambda *a, **k: logs.append(" ".join(str(x) for x in a))
-    rt2.load_checkpoint(str(path))                                     # the unmodified loader
-    assert not any("[WARN]" in m for m in logs), logs
-    assert any("loaded EMA" in m for m in logs), logs
-    assert rt2.epoch == 3 and rt2.global_step == tr.global_step
-    assert abs(rt2.model.mean_density - tr.mean_density.item()) < 1e-7
-    for n, a, b in zip(names, rt2.ema.shadow_params, st["shadow_params"]):
-        assert torch.equal(a, b.to(a.device)), n
-    assert torch.equal(rt2.model.density_bitfield, tr.density_bitfield)
+    ck = torch.load(str(path), map_location="cuda")
+    assert {k: list(v.shape) for k, v in ck["model"].items()} == json.loads(G[P + "state_dict"])
+    assert len(ck["ema"]["shadow_params"]) == len(names) and ck["ema"]["num_updates"] == 3
+    for (n, shape), a, b in zip(params, ck["ema"]["shadow_params"], st["shadow_params"]):
+        assert list(a.shape) == shape and torch.equal(a, b.to(a.device)), n
+    assert {"stats", "epoch", "global_step"} <= set(ck)          # read unconditionally by the loader (utils.py:1449-1451)
+    assert ck["epoch"] == 3 and ck["global_step"] == tr.global_step
+    assert abs(ck["mean_density"] - tr.mean_density.item()) < 1e-7
+    assert torch.equal(ck["model"]["density_bitfield"], tr.density_bitfield)
+    # --- the reference model loaded from our checkpoint of the seeded parameters renders what we render ---
+    t2 = _handoff_checkpoint(tmp_path / "seeded.pth")
     ro, rd = cases.rays(2048, seed=21)
-    with torch.no_grad():
-        rt2.model.eval()
-        ev = rt2.model.render(ro.cuda(), rd.cuda(), bg_color=1, perturb=False,
-                              **{k: v for k, v in vars(opt).items() if k not in ("bg_color", "perturb")})
-    img, ws, _ = tr.render(ro.cuda(), rd.cuda(), bg_color=1.0)
-    assert (img - ev["image"]).abs().max().item() <= 2e-3
+    img, ws, _ = t2.render(ro.cuda(), rd.cuda(), bg_color=1.0)
+    a, r = G.take(P + "image", img)
+    assert (a - r).abs().max().item() <= 2e-3
 
 
-@pytest.mark.parametrize("name", ["lego", "garden"])
-def test_mark_untrained_grid_matches_reference(name):
-    """SURVEY.md section 8 f2: Stage0Trainer.mark_untrained_grid (one kernel, csrc/grid_aux.cu) vs the unmodified
-    NeRFRenderer.mark_untrained_grid (renderer.py:985-1071) on the same camera set; cells may differ only where a frustum plane
-    passes within fp32 rounding of the cell position (the reference's batched matmul and the kernel round differently)."""
-    import types
+def _untrained_setup(name):
     c = CASES[name]
-    ref_stage, ns = _ref_stack()
     poses = S.orbit_cameras(23, radius=c["radius"], seed=4)
-    intr = S.lego_intrinsics()
     cnf = None
     if c["cam_nf"]:
         d = poses[:, :3, 3].norm(dim=-1)
         cnf = torch.stack([(d - 1.0).clamp(min=0.05), d + 14.0], -1)
+    return c, poses, S.lego_intrinsics(), cnf
+
+
+def _reference_mark_untrained(G, name):
+    import types
+    ref_stage, ns = _ref_stack()
+    c, poses, intr, cnf = _untrained_setup(name)
     opt = ref_stage.default_opt(bound=c["bound"], dt_gamma=c["dt_gamma"], adaptive_num_rays=False)
     model = ns.make_model(opt).cuda()
     dataset = types.SimpleNamespace(poses=poses.numpy(), intrinsics=intr)
@@ -567,11 +693,25 @@ def test_mark_untrained_grid_matches_reference(name):
         dataset.cam_near_far = cnf.cuda()
     with ns.context():
         model.mark_untrained_grid(dataset)
-    ref = model.density_grid < 0
+    ref = (model.density_grid < 0).cpu().numpy()
+    G.put(f"mark_untrained/{name}/shape", np.array(ref.shape))
+    G.put(f"mark_untrained/{name}/bits", np.packbits(ref.reshape(-1)))
+
+
+@pytest.mark.parametrize("name", ["lego", "garden"])
+def test_mark_untrained_grid_matches_reference(name):
+    """SURVEY.md section 8 f2: Stage0Trainer.mark_untrained_grid (one kernel, csrc/grid_aux.cu) vs the unmodified
+    NeRFRenderer.mark_untrained_grid (renderer.py:985-1071) on the same camera set; cells may differ only where a frustum plane
+    passes within fp32 rounding of the cell position (the reference's batched matmul and the kernel round differently)."""
+    G = gold()
+    c, poses, intr, cnf = _untrained_setup(name)
+    shape = tuple(G[f"mark_untrained/{name}/shape"])
+    ref = torch.from_numpy(np.unpackbits(G[f"mark_untrained/{name}/bits"])[:int(np.prod(shape))].astype(bool)).reshape(shape).cuda()
     cfg = Stage0Config(bound=c["bound"], dt_gamma=c["dt_gamma"], num_rays=128, max_samples=128 * 128)
     tr = Stage0Trainer(cfg, seed=0)
     cnt = tr.mark_untrained_grid(poses, intr, cnf)
     ours = tr.density_grid < 0
+    assert ours.shape == ref.shape
     assert int(cnt.item()) == int(ours.sum().item())
     frac_marked = ref.float().mean().item()
     if c["bound"] > 1:          # (orbit cameras looking at the origin see every cell of the bound-1 cube: nothing is marked there)
@@ -583,17 +723,12 @@ def test_mark_untrained_grid_matches_reference(name):
         assert abs(ours[cas].float().mean().item() - ref[cas].float().mean().item()) < 1e-4
 
 
-@pytest.mark.parametrize("name", ["lego", "garden"])
-def test_tv_gradient_alone_matches_reference_post_train_step(name):
-    """The TV gradient of one 4096-ray batch in isolation: Stage0Trainer.tv() (one launch, per-lane weight lambda or 10 lambda, runs of
-    same-cell lanes evaluated once) vs the UNMODIFIED Trainer.post_train_step (utils.py:801-823: one or two calls of
-    GridEncoder.grad_total_variation on the marched positions) on a zeroed gradient."""
+def _tv_setup(name):
+    """ours with the seeded parameters, one batch marched; -> (c, tr, M, marched positions through the C ABI in ray order)"""
     c = CASES[name]
-    ref_stage, ns = _ref_stack()
     grid, bits, bricks = _scene(c)
     tr = _make_ours(c, bits, grid)
-    _warm_up(tr, c, bricks, steps=20)
-    rt = _ref_trainer(ref_stage, ns, c, tr.export_reference_state(), True)
+    refcall.seeded_state(tr)
     ro, rd = _batch(c, 7)
     cnf = _cam_nf(c, ro)
     g = torch.Generator().manual_seed(3)
@@ -602,8 +737,7 @@ def test_tv_gradient_alone_matches_reference_post_train_step(name):
     tr.march()
     torch.cuda.synchronize()
     M = int(tr.counters[1].item())
-    # the marched positions, through the reference's own operator (bit-exact with ours)
-    rm = ns.raymarching
+    from nerf2mesh_b200 import raymarching as rm
     aabb = torch.tensor([-c["bound"]] * 3 + [c["bound"]] * 3, device="cuda")
     nears, fars = rm.near_far_from_aabb(tr.rays_o, tr.rays_d, aabb, 0.05)
     if cnf is not None:
@@ -617,14 +751,37 @@ def test_tv_gradient_alone_matches_reference_post_train_step(name):
     assert int(counter.item()) == M
     xyzs = torch.zeros(M, 3, device="cuda"); dirs = torch.zeros(M, 3, device="cuda"); ts = torch.zeros(M, 2, device="cuda")
     call("n2m_march_rays_train", *args, ptr(xyzs), ptr(dirs), ptr(ts), ptr(rays), ptr(counter), ptr(tr.noises), ptr(tbuf), stream())
-    # reference: post_train_step on a zero gradient
+    torch.cuda.synchronize()
+    return c, tr, M, xyzs
+
+
+def _reference_tv_gradient(G, name):
+    ref_stage, ns = _ref_stack()
+    c, tr, M, xyzs = _tv_setup(name)
+    rt = _ref_trainer(ref_stage, ns, c, tr.export_reference_state(), True)
+    # reference: post_train_step on a zero gradient, on the marched positions (the reference's operator is bit-exact with ours)
     for p_ in rt.model.parameters():
         p_.grad = torch.zeros_like(p_)
     rt.tmp_xyzs = xyzs
     rt.scaler = torch.amp.GradScaler("cuda", enabled=False)          # unscale_ of an untouched scaler would raise; TV itself is unscaled
     rt.post_train_step()
     g_ref = rt.model.encoder.embeddings.grad.reshape(-1)
-    # ours
+    offs = _levels(tr)
+    G.put(f"tv/{name}/M", M)
+    for l in range(16):
+        g = g_ref[offs[l]:offs[l + 1]]
+        G.put(f"tv/{name}/level{l}", g, index=refcall.support_rows(g, k=K_LEVEL, key=f"tv/{name}/level{l}"))
+
+
+@pytest.mark.parametrize("name", ["lego", "garden"])
+def test_tv_gradient_alone_matches_reference_post_train_step(name):
+    """The TV gradient of one 4096-ray batch in isolation: Stage0Trainer.tv() (one launch, per-lane weight lambda or 10 lambda, runs of
+    same-cell lanes evaluated once) vs the UNMODIFIED Trainer.post_train_step (utils.py:801-823: one or two calls of
+    GridEncoder.grad_total_variation on the marched positions) on a zeroed gradient; per level on the stored rows (a sample of the rows the
+    reference's gradient reaches; all of them where they are few, as at the coarse levels)."""
+    G = gold()
+    c, tr, M, xyzs = _tv_setup(name)
+    assert M == G[f"tv/{name}/M"]
     tr.gtable.zero_()
     tr.tv()
     torch.cuda.synchronize()
@@ -633,31 +790,29 @@ def test_tv_gradient_alone_matches_reference_post_train_step(name):
     assert tr.counters[15].item() == n_out and tr.counters[3].item() == M - n_out
     if c["bound"] > 1:
         assert n_out > 1000 and M - n_out > 1000
-    offs = tr.offsets.cpu().tolist()
-    worst = 0.0
+    offs = _levels(tr)
     for l in range(16):
-        a, r = g_ours[offs[l]:offs[l + 1]].double(), g_ref[offs[l]:offs[l + 1]].double()
-        sc = r.abs().max().item()
+        key = f"tv/{name}/level{l}"
+        a, r = G.take(key, g_ours[offs[l]:offs[l + 1]])
+        sc = G[key + ":absmax"]
         assert sc > 0, l
         rel = ((a - r).norm() / r.norm()).item()
-        worst = max(worst, rel)
         # the coarse, dense levels receive ~1e5 equal fp32 atomicAdd increments per cell in the reference, whose rounding drifts one way
         # (|ours| / |ref| = 1.001 measured at level 1 of the garden batch, DESIGN.md section 2); ours adds merged runs
         tol = 3e-3 if l < 4 else 1e-3
         assert rel <= tol, (l, rel, (a - r).abs().max().item(), sc, (a.norm() / r.norm()).item())
 
 
-def test_density_volume_matches_reference_export_stage0_input():
-    """SURVEY.md section 8 f4: the marching-cubes input of NeRFRenderer.export_stage0 (renderer.py:480-513) -- sigma on a regular grid
-    times the occupancy mask -- from Stage0Trainer.density_volume vs the same lines evaluated with the unmodified reference model."""
+def _reference_density_volume(G):
+    """the marching-cubes input of NeRFRenderer.export_stage0 (renderer.py:480-513) -- sigma on a regular grid times the occupancy
+    mask -- evaluated with the unmodified reference model, verbatim structure"""
     import torch.nn.functional as F
-    c, tr, rt, bricks = _trained_pair("lego", steps=24)
+    c, tr, rt, bricks = _seeded_pair("lego")
     torch.manual_seed(5)
     tr.update_density_grid()
     rt.model.density_grid.copy_(tr.density_grid); rt.model.mean_density = float(tr.mean_density.item())
     model, R, S_ = rt.model, 96, 48
     ns = rt.ns
-    # renderer.py:480-513, verbatim structure
     density_thresh = min(model.mean_density, model.density_thresh)
     sigmas = torch.zeros([R] * 3, dtype=torch.float32, device="cuda")
     X = torch.linspace(-1, 1, R).split(S_); Y = torch.linspace(-1, 1, R).split(S_); Z = torch.linspace(-1, 1, R).split(S_)
@@ -674,11 +829,41 @@ def test_density_volume_matches_reference_export_stage0_input():
     mask[tuple(all_coords.T)] = model.density_grid[0]
     mask = F.interpolate(mask.unsqueeze(0).unsqueeze(0), size=[R] * 3, mode="nearest").squeeze(0).squeeze(0)
     ref = torch.nan_to_num(sigmas * (mask > density_thresh), 0)
-    ours = tr.density_volume(R, density_thresh=model.density_thresh)
-    assert ours.shape == ref.shape and (ref > 0).float().mean().item() > 0.01
-    assert torch.equal(ours > 0, ref > 0)
-    assert (ours - ref).abs().max().item() <= 2e-3 * ref.abs().max().item()
-    # R == grid_size: the density grid itself, re-mapped from Morton order (renderer.py:484-488)
+    G.put("density_volume/volume", ref, 3072)
+    G.put("density_volume/positive", refcall.digest(ref > 0))
+    G.put("density_volume/positive_fraction", (ref > 0).float().mean().item())
+
+
+def test_density_volume_matches_reference_export_stage0_input():
+    """SURVEY.md section 8 f4: the marching-cubes input of NeRFRenderer.export_stage0 (renderer.py:480-513) -- sigma on a regular grid
+    times the occupancy mask -- from Stage0Trainer.density_volume vs the same lines evaluated with the unmodified reference model."""
+    from nerf2mesh_b200 import raymarching as rm
+    G = gold()
+    c, tr, bricks = _seeded("lego")
+    torch.manual_seed(5)
+    tr.update_density_grid()
+    ours = tr.density_volume(96, density_thresh=10.0)
+    assert ours.shape == (96, 96, 96) and G["density_volume/positive_fraction"] > 0.01
+    assert refcall.digest(ours > 0) == G["density_volume/positive"]
+    a, r = G.take("density_volume/volume", ours)
+    assert (a - r).abs().max().item() <= 2e-3 * G["density_volume/volume:absmax"]
+    # R == grid_size: the density grid itself, re-mapped from Morton order (renderer.py:484-488).  The expectation uses our own
+    # morton3D_invert, so it is not independent of the code under test; that operator is pinned bit-exact against the reference's in
+    # test_gpu_raymarching.py::test_packbits_morton_flatten_exact
     g = tr.density_volume(128)
-    ref_g = torch.zeros([128] * 3, device="cuda"); ref_g[tuple(all_coords.T)] = model.density_grid[0]
+    all_coords = rm.morton3D_invert(torch.arange(128 ** 3, device="cuda", dtype=torch.int)).long()
+    ref_g = torch.zeros([128] * 3, device="cuda"); ref_g[tuple(all_coords.T)] = tr.density_grid[0]
     assert torch.equal(g, torch.nan_to_num(ref_g, 0))
+
+
+def reference_outputs(G, tmp_dir):
+    """run the reference side of every test above that has one (needs oracle/_ref and the staged reference Python files) into G"""
+    for name in ("lego", "garden", "garden_notv"):
+        _reference_fused_step(G, name)
+    for name in ("lego", "garden"):
+        _reference_density_grid_update(G, name)
+        _reference_mark_untrained(G, name)
+        _reference_tv_gradient(G, name)
+    _reference_evaluation_render(G)
+    _reference_checkpoint(G, tmp_dir)
+    _reference_density_volume(G)

@@ -493,11 +493,7 @@ def test_reference_state_dict_and_checkpoint_schema(tmp_path):
         assert torch.equal(v, s2[k]), k
 
 
-def test_tv_random_point_fallback(ref_gridencoder):
-    """GridEncoder.grad_total_variation's fallback (grid.py:181-183, reached from utils.py:815-823 when a TV call gets no sample): the
-    fused path evaluates the same TV gradient at its own hash-generated points; fed to the REFERENCE kernel, those points give the same
-    gradient.  And the fallback fires exactly for the groups the TV pass counted as empty."""
-    import numpy as np
+def _tv_fallback_points():
     tr, b = make(N=96)
     stage(tr, b)
     tr.tv_fallback_points = 20000
@@ -507,17 +503,41 @@ def test_tv_random_point_fallback(ref_gridencoder):
     tr.gtable.zero_()
     tr.tv_random(dump=pts)                      # test hook: unconditional, weight lambda_tv
     torch.cuda.synchronize()
-    assert pts.min().item() >= 0 and pts.max().item() < 1 and abs(pts.mean().item() - 0.5) < 0.01
-    ours = tr.export_reference_grads()["encoder.embeddings"]
+    return tr, pts
+
+
+def reference_outputs(G):
+    """the REFERENCE kernel's TV gradient at the fallback points (tests/golden/make_golden.py; needs oracle/_ref)"""
+    import numpy as np
+    import refcall
+    from oracle.build_ref import load_ref
+    tr, pts = _tv_fallback_points()
     st = tr.export_reference_state()
     emb = st["encoder.embeddings"].contiguous()
     grad = torch.zeros_like(emb)
     S_ = float(np.log2(tr.cfg.per_level_scale))
-    ref_gridencoder.grad_total_variation(pts, emb, grad, tr.offsets, tr.cfg.lambda_tv, pts.shape[0], 3, 1, 16, S_, 16, 0, False)
+    load_ref("_ref_gridencoder").grad_total_variation(pts, emb, grad, tr.offsets, tr.cfg.lambda_tv, pts.shape[0], 3, 1, 16, S_, 16, 0, False)
     torch.cuda.synchronize()
-    scale = grad.abs().max().item()
+    G.put("tv_fallback/points", refcall.digest(pts))
+    G.put("tv_fallback/grad", grad, index=refcall.support_rows(grad, k=2048, key="tv_fallback/grad"))
+
+
+def test_tv_random_point_fallback():
+    """GridEncoder.grad_total_variation's fallback (grid.py:181-183, reached from utils.py:815-823 when a TV call gets no sample): the
+    fused path evaluates the same TV gradient at its own hash-generated points; fed to the REFERENCE kernel, those points give the same
+    gradient (stored in tests/golden/reference_model.npz, on a seeded sample of the rows it reaches).  And the fallback fires exactly for
+    the groups the TV pass counted as empty."""
+    import os
+    import refcall
+    tr, pts = _tv_fallback_points()
+    assert pts.min().item() >= 0 and pts.max().item() < 1 and abs(pts.mean().item() - 0.5) < 0.01
+    ours = tr.export_reference_grads()["encoder.embeddings"]
+    G = refcall.Golden(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_model.npz"))
+    assert refcall.digest(pts) == G["tv_fallback/points"], "the stored reference gradient belongs to another point set"
+    scale = G["tv_fallback/grad:absmax"]
     assert scale > 0
-    assert (ours - grad).abs().max().item() <= 1e-4 * scale, ((ours - grad).abs().max().item(), scale)
+    a, r = G.take("tv_fallback/grad", ours)
+    assert (a - r).abs().max().item() <= 1e-4 * scale, ((a - r).abs().max().item(), scale)
     # a new point set every optimizer step
     pts2 = torch.zeros_like(pts)
     tr.opt_state[2] += 1

@@ -3,11 +3,20 @@ kernels) against the reference's render_stage1 arithmetic composed from the UNMO
 network.py:170-189, over the reference's grid-encoder kernels) and torch ops, following nerf/renderer.py:824-907 and
 nerf/utils.py:703-712 line by line -- with this repo's rasterize / interpolate standing in for nvdiffrast (itself checked against the
 CPU oracle in test_gpu_raster.py), without dr.antialias and with this repo's antialias (csrc/antialias.cu, checked against its CPU oracle
-in test_gpu_antialias.py) in the place of the library's, including the image-loss gradient it sends to the vertices."""
+in test_gpu_antialias.py) in the place of the library's, including the image-loss gradient it sends to the vertices.
+
+The reference's results are stored in tests/golden/reference_stage1.npz (refcall.Golden: scalars, digests, and for every large tensor its
+values at stored rows -- a seeded sample, or for the sparse colour-table gradient a sample of the rows it reaches -- with its full-tensor
+size, max |.| and norm); `reference_outputs()` below regenerates them where the
+reference is available (tests/golden/make_golden.py).  A comparison with a sampled tensor is made on its stored rows."""
+import os
+
 import numpy as np
 import pytest
 import torch
 import torch.nn.functional as F
+
+import refcall
 
 from nerf2mesh_b200 import raster as dr
 from nerf2mesh_b200 import synthetic as S
@@ -18,8 +27,20 @@ from oracle import raster_oracle as R
 
 pytestmark = pytest.mark.gpu
 
+GOLD_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_stage1.npz")
+K_IMG, K_GRAD = 768, 1024
+COLOR_GRADS = ["encoder_color.embeddings"] + [n for n, _ in MLP_LAYOUT if not n.startswith("sigma")]
+STAGE1_CASES = [(2, False), (1, False), (2, True), (1, True)]
+_GOLD = []
 
-def _setup(h0=96, w0=96, ssaa=2, steps=30, antialias=False, subdiv=4, **s1_kw):
+
+def gold():
+    if not _GOLD:
+        _GOLD.append(refcall.Golden(GOLD_PATH))
+    return _GOLD[0]
+
+
+def _setup(h0=96, w0=96, ssaa=2, steps=30, antialias=False, subdiv=4, seeded=False, **s1_kw):
     N = 1024
     cfg = Stage0Config(bound=1.0, num_rays=N, max_samples=N * 256)
     t0 = Stage0Trainer(cfg, seed=5)
@@ -27,6 +48,9 @@ def _setup(h0=96, w0=96, ssaa=2, steps=30, antialias=False, subdiv=4, **s1_kw):
     t0.set_occupancy(bits, grid)
     g = torch.Generator().manual_seed(0)
     poses = S.orbit_cameras(100, seed=0)
+    if seeded:          # parameters that depend on a seed alone, for the comparisons with stored reference results
+        refcall.seeded_state(t0)
+        steps = 0
     for it in range(steps):       # non-trivial colour parameters
         ro, rd, _, _ = S.sample_rays(poses, S.lego_intrinsics(), 800, 800, N, g)
         t0.step(ro, rd, S.render_bricks(ro, rd, bricks), torch.rand(N, 3, generator=g), torch.rand(N, generator=g), use_graph=False)
@@ -97,42 +121,66 @@ def _reference_stage1(ns, ref_stage, t0, s1, mvp, rays_d, gt, bg, lambda_mask=0.
                 grad_vertices=None if vertices.grad is None else vertices.grad * inv)
 
 
-@pytest.mark.parametrize("ssaa,antialias", [(2, False), (1, False), (2, True), (1, True)])
-def test_stage1_step_matches_reference_composition(ssaa, antialias):
+def _ref_ns():
     from oracle import ref_stage
     if not ref_stage.staged():
         pytest.skip("reference Python files not staged")
-    ns = ref_stage.load("ref")
+    return ref_stage, ref_stage.load("ref")
+
+
+def _step_setup(ssaa, antialias):
     # antialias only sees the edges of the foreground pixel's own triangle: on the 5120-face sphere (facets a few pixels wide, slivers at
     # the limb) it blends a handful of outline pixels (3-5 measured), so the antialiased cases use the 320-face sphere
-    t0, s1, mvp, rays_d, gt, bg = _setup(ssaa=ssaa, antialias=antialias, subdiv=2 if antialias else 4)
+    t0, s1, mvp, rays_d, gt, bg = _setup(ssaa=ssaa, antialias=antialias, subdiv=2 if antialias else 4, seeded=True)
     t0.opt_state[0] = 4096.0
+    return t0, s1, mvp, rays_d, gt, bg
+
+
+def _reference_step(G, ssaa, antialias):
+    P = f"step/{ssaa}/{antialias}/"
+    ref_stage, ns = _ref_ns()
+    t0, s1, mvp, rays_d, gt, bg = _step_setup(ssaa, antialias)
     ref = _reference_stage1(ns, ref_stage, t0, s1, mvp, rays_d, gt, bg, antialias=antialias)
+    G.put(P + "covered", ref["covered"]); G.put(P + "rast", refcall.digest(ref["rast"])); G.put(P + "loss", ref["loss"])
+    G.put(P + "image", ref["image"], K_IMG); G.put(P + "ws", ref["ws"], K_IMG)
+    if antialias:
+        G.put(P + "grad_vertices", ref["grad_vertices"].cpu().numpy())
+    for name in COLOR_GRADS:          # the colour table's gradient is sparse: stored at a sample of the rows it reaches
+        g, key = ref["grads"][name], P + f"grad/{name}"
+        G.put(key, g, index=refcall.support_rows(g, k=K_GRAD, key=key) if name == "encoder_color.embeddings" else refcall.sample_index(g.numel(), K_GRAD, key))
+
+
+@pytest.mark.parametrize("ssaa,antialias", STAGE1_CASES)
+def test_stage1_step_matches_reference_composition(ssaa, antialias):
+    P = f"step/{ssaa}/{antialias}/"
+    G = gold()
+    t0, s1, mvp, rays_d, gt, bg = _step_setup(ssaa, antialias)
     t0.gtable.zero_(); t0.g_mlp.zero_()
     s1.forward(mvp, rays_d)
     s1.loss_backward(gt, bg)
     torch.cuda.synchronize()
-    assert s1.counters[2].item() == 0 and s1.counters[1].item() == ref["covered"] and ref["covered"] > 0.1 * s1.h * s1.w
-    assert torch.equal(s1.rast, ref["rast"])
-    assert (s1.image - ref["image"]).abs().max().item() <= 2e-3
-    assert (s1.weights_sum - ref["ws"]).abs().max().item() <= (1e-5 if antialias else 1e-6)
+    covered = G[P + "covered"]
+    assert s1.counters[2].item() == 0 and s1.counters[1].item() == covered and covered > 0.1 * s1.h * s1.w
+    assert refcall.digest(s1.rast) == G[P + "rast"]
+    a, r = G.take(P + "image", s1.image)
+    assert (a - r).abs().max().item() <= 2e-3
+    a, r = G.take(P + "ws", s1.weights_sum)
+    assert (a - r).abs().max().item() <= (1e-5 if antialias else 1e-6)
     if antialias:
         # the silhouette pixels changed, and the loss reaches the vertices through them (the reference's only path to vertices_offsets)
         assert ((s1.aa[:, 3] - s1.rgba[:, 3]).abs() > 1e-3).sum().item() > 30
-        gv, rv = s1.vertex_gradient().double().flatten(), ref["grad_vertices"].double().flatten()
+        gv, rv = s1.vertex_gradient().double().flatten().cpu(), torch.from_numpy(G[P + "grad_vertices"]).double().flatten()
         assert rv.abs().max().item() > 0
         cos = (torch.dot(gv, rv) / (gv.norm() * rv.norm() + 1e-300)).item()
         assert cos > 0.999 and ((gv - rv).norm() / rv.norm()).item() <= 3e-2, (cos, ((gv - rv).norm() / rv.norm()).item())
-    assert abs(s1.read_loss() - ref["loss"]) <= 1e-3 * abs(ref["loss"])
+    ref_loss = G[P + "loss"]
+    assert abs(s1.read_loss() - ref_loss) <= 1e-3 * abs(ref_loss)
     g = t0.export_reference_grads()
     assert t0.opt_state[3].item() == 0
-    for name in ["encoder_color.embeddings"] + [n for n, _ in MLP_LAYOUT if not n.startswith("sigma")]:
-        a, r = g[name].double().flatten(), ref["grads"][name].double().flatten()
-        scale = r.abs().max().item()
-        assert scale > 0, name
-        cos = (torch.dot(a, r) / (a.norm() * r.norm() + 1e-300)).item()
-        rel = ((a - r).norm() / r.norm()).item()
-        assert cos > 0.9995 and rel <= 3e-2, (name, cos, rel)
+    for name in COLOR_GRADS:
+        assert G[P + f"grad/{name}:absmax"] > 0, name
+        e = G.cmp(P + f"grad/{name}", g[name])
+        assert e["cos"] > 0.9995 and e["rel_l2"] <= 3e-2, (name, e)
     # the density branch receives no gradient in stage 1
     assert g["encoder.embeddings"].abs().max().item() == 0
     assert g["sigma_net.net.0.weight"].abs().max().item() == 0 and g["sigma_net.net.1.weight"].abs().max().item() == 0
@@ -181,37 +229,54 @@ def test_graph_replayed_step_equals_eager_step():
     assert len(s1._graphs) == 1 and abs(s1.read_loss() - loss_e) <= 1e-6 * abs(loss_e)
 
 
-def test_vertex_offset_optimizer_matches_autograd_and_torch_adam():
-    """lr_vert > 0: the `vertices_offsets` group of the reference's stage 1 (renderer.py:160,180; regularisers utils.py:750-779).  The total
-    gradient = image loss through dr.antialias (reference composition) + lambda_lap * laplacian_smooth_loss (the reference's own function)
-    + lambda_offsets * mean(sum(offsets^2)) by autograd; the update = torch.optim.Adam(lr_vert, eps=1e-15) on that gradient."""
-    from oracle import ref_stage
-    if not ref_stage.staged():
-        pytest.skip("reference Python files not staged")
-    ns = ref_stage.load("ref")
-    lam_lap, lam_off, lr_v = 0.01, 0.1, 1e-3
-    t0, s1, mvp, rays_d, gt, bg = _setup(ssaa=2, antialias=True, subdiv=2, steps=8, lr_vert=lr_v, lambda_lap=lam_lap, lambda_offsets=lam_off)
+LAM_LAP, LAM_OFF, LR_V = 0.01, 0.1, 1e-3
+
+
+def _vertex_setup():
+    t0, s1, mvp, rays_d, gt, bg = _setup(ssaa=2, antialias=True, subdiv=2, seeded=True, lr_vert=LR_V, lambda_lap=LAM_LAP, lambda_offsets=LAM_OFF)
     t0.opt_state[0] = 4096.0
     g = torch.Generator(device="cuda").manual_seed(3)
     s1.offsets.copy_(torch.randn(s1.offsets.shape, device="cuda", generator=g) * 2e-3)
     s1.vertices.copy_(s1.base_vertices + s1.offsets)
-    off_old = s1.offsets.clone()
-    ref = _reference_stage1(ns, ref_stage, t0, s1, mvp, rays_d, gt, bg, antialias=True)            # image loss + its gradient w.r.t. the vertices
-    off = off_old.clone().requires_grad_(True)
-    reg = lam_lap * ns.utils.laplacian_smooth_loss(s1.base_vertices + off, s1.triangles) + lam_off * (off ** 2).sum(-1).mean()
+    return t0, s1, mvp, rays_d, gt, bg
+
+
+def _reference_vertex_offsets(G):
+    """image loss + its gradient w.r.t. the vertices (reference composition), and the regularisers through the reference's own
+    laplacian_smooth_loss with their gradient w.r.t. the offsets by autograd"""
+    ref_stage, ns = _ref_ns()
+    t0, s1, mvp, rays_d, gt, bg = _vertex_setup()
+    ref = _reference_stage1(ns, ref_stage, t0, s1, mvp, rays_d, gt, bg, antialias=True)
+    off = s1.offsets.clone().requires_grad_(True)
+    reg = LAM_LAP * ns.utils.laplacian_smooth_loss(s1.base_vertices + off, s1.triangles) + LAM_OFF * (off ** 2).sum(-1).mean()
     reg.backward()
+    G.put("vertex/loss", ref["loss"]); G.put("vertex/grad_vertices", ref["grad_vertices"].cpu().numpy())
+    G.put("vertex/reg", float(reg)); G.put("vertex/grad_reg", off.grad.cpu().numpy())
+
+
+def test_vertex_offset_optimizer_matches_autograd_and_torch_adam():
+    """lr_vert > 0: the `vertices_offsets` group of the reference's stage 1 (renderer.py:160,180; regularisers utils.py:750-779).  The total
+    gradient = image loss through dr.antialias (reference composition) + lambda_lap * laplacian_smooth_loss (the reference's own function)
+    + lambda_offsets * mean(sum(offsets^2)) by autograd; the update = torch.optim.Adam(lr_vert, eps=1e-15) on that gradient."""
+    G = gold()
+    lr_v = LR_V
+    t0, s1, mvp, rays_d, gt, bg = _vertex_setup()
+    off_old = s1.offsets.clone()
+    ref_loss, reg = G["vertex/loss"], G["vertex/reg"]
+    ref_gv = torch.from_numpy(G["vertex/grad_vertices"]).cuda()
+    off_grad = torch.from_numpy(G["vertex/grad_reg"]).cuda()
     t0.gtable.zero_(); t0.g_mlp.zero_()
     s1.step(mvp, rays_d, gt, bg)
     torch.cuda.synchronize()
     assert t0.opt_state[3].item() == 0
-    assert abs(s1.read_loss() - (ref["loss"] + float(reg))) <= 1e-3 * abs(ref["loss"] + float(reg))
+    assert abs(s1.read_loss() - (ref_loss + reg)) <= 1e-3 * abs(ref_loss + reg)
     img_part = s1.vertex_gradient()
     reg_part = s1.grad_offsets - img_part
-    assert ((reg_part - off.grad).norm() / off.grad.norm()).item() <= 1e-4, ((reg_part - off.grad).norm() / off.grad.norm()).item()
-    tot_ref = ref["grad_vertices"] + off.grad
+    assert ((reg_part - off_grad).norm() / off_grad.norm()).item() <= 1e-4, ((reg_part - off_grad).norm() / off_grad.norm()).item()
+    tot_ref = ref_gv + off_grad
     rel = ((s1.grad_offsets - tot_ref).norm() / tot_ref.norm()).item()
     assert rel <= 3e-2, rel
-    assert img_part.abs().max().item() > 0 and (ref["grad_vertices"].norm() / off.grad.norm()).item() > 1e-3      # both parts matter in the sum
+    assert img_part.abs().max().item() > 0 and (ref_gv.norm() / off_grad.norm()).item() > 1e-3      # both parts matter in the sum
     # Adam: torch's optimizer fed with OUR gradients, two steps (fresh state, as the reference's stage-1 trainer starts)
     p = torch.nn.Parameter(off_old.clone())
     opt = torch.optim.Adam([p], lr=lr_v, eps=1e-15)
@@ -233,3 +298,10 @@ def test_vertex_offset_optimizer_matches_autograd_and_torch_adam():
     t0.adam(between=s1._vertex_step)
     torch.cuda.synchronize()
     assert torch.equal(s1.offsets, before) and s1.vert_state[0].item() == 2 and t0.opt_state[0].item() == 0.5 * scale
+
+
+def reference_outputs(G):
+    """run the reference side of the tests above that have one (needs oracle/_ref and the staged reference Python files) into G"""
+    for ssaa, antialias in STAGE1_CASES:
+        _reference_step(G, ssaa, antialias)
+    _reference_vertex_offsets(G)

@@ -2,6 +2,8 @@
 import ctypes
 import os
 import re
+import subprocess
+import sys
 
 import numpy as np
 import torch
@@ -41,7 +43,10 @@ def test_library_exports_every_declared_symbol():
     for s in syms:
         assert hasattr(_lib.lib, s), f"libn2m_b200.so does not export {s}"
     assert _lib.lib.n2m_version() == 100
-    assert _lib.last_error() == ""
+    # loading leaves no error message: checked in a fresh interpreter, since tests that run earlier in this one provoke errors on purpose
+    r = subprocess.run([sys.executable, "-c", "from nerf2mesh_b200 import _lib; print(repr(_lib.last_error()))"], cwd=ROOT,
+                       capture_output=True, text=True)
+    assert r.returncode == 0 and r.stdout.strip() == "''", (r.stdout, r.stderr[-500:])
 
 
 def test_bindings_cover_the_headers():
